@@ -26,6 +26,10 @@ schedules partitions independently), one per GPU, no data-path exchange -- weak 
 sweep of every batch split across the N GPUs and exchanged peer-to-peer (strong scaling of config 3), every rank checked
 against the oracle and against each other.
 `--impl reference` times the CPU port alone, same metric / config.
+`--dump-outputs DIR` writes the bindings of the headline arm's last timed step as DIR/ask.npy and DIR/node.npy (float64, in
+commit order; rank 0's partition at N > 1): the inputs are seeded, so two builds run with the same arguments can be compared
+output for output.
+The benchmark writes nothing into the source tree, which may be read-only: what it compiles goes to a temporary directory.
 """
 from __future__ import annotations
 
@@ -33,12 +37,15 @@ import argparse
 import ctypes as C
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True     # no __pycache__ next to the modules imported from the tree
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -249,17 +256,28 @@ class Arm:
         self.eng.close()
 
 
+_CPU_ENGINE = None
+
+
+def cpu_engine_lib():
+    """tests/host/engine_shim.cpp, compiled once per run from the current sources into a temporary directory"""
+    global _CPU_ENGINE
+    if _CPU_ENGINE is None:
+        tmp = tempfile.mkdtemp(prefix="yk_bench_")
+        try:
+            so = os.path.join(tmp, "engine_shim.so")
+            subprocess.check_call(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-fPIC", "-shared", "-pthread", "-w", "-o", so,
+                                   os.path.join(ROOT, "tests", "host", "engine_shim.cpp")])
+            _CPU_ENGINE = C.CDLL(so)      # stays mapped once its file is gone
+        finally:
+            shutil.rmtree(tmp, ignore_errors=True)
+    return _CPU_ENGINE
+
+
 def cpu_engine_time(snap, threads, reps=2, batch=4096):
     """the same ordering engine + ordered commit with the sweep on the host cores (tests/host/engine_shim.cpp)"""
     from test_engine_host import run_engine_host
-    so = os.path.join(ROOT, "tests", "host", "_build", "engine_shim.so")
-    src = os.path.join(ROOT, "tests", "host", "engine_shim.cpp")
-    csrc = os.path.join(ROOT, "yunikorn_k8shim_b200", "csrc")
-    newest = max([os.path.getmtime(src)] + [os.path.getmtime(os.path.join(csrc, f)) for f in os.listdir(csrc) if f.endswith((".h", ".hpp"))])
-    if not os.path.exists(so) or os.path.getmtime(so) < newest:
-        os.makedirs(os.path.dirname(so), exist_ok=True)
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-fPIC", "-shared", "-pthread", "-w", "-o", so, src])
-    lib = C.CDLL(so)
+    lib = cpu_engine_lib()
     lib.host_set_bench_mode(C.c_int(threads), C.c_int(1))
     best, ask, node = 1e18, None, None
     # epoch length: the engine's general rule (5/8 of the nodes) and its few-signature rule (one epoch): the better of the two
@@ -328,7 +346,13 @@ def main():
     ap.add_argument("--quick", action="store_true", help="headline arm only (no side workloads, no CPU arms)")
     ap.add_argument("--no-row-sharing", action="store_true",
                     help="sweep one row per ask even when asks have identical predicate inputs (YK_FLAG_NO_ROW_SHARING)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the bindings of the headline arm's last timed step to DIR/ask.npy and DIR/node.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the engine computed: it needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     args.workload = {"0": "config2", "2": "config2", "3": "config3", "4": "config4", "5": "config5", "reference": "reference_shape"}[str(args.config)]
     if args.masks:
@@ -368,6 +392,10 @@ def main():
     want = oc.run(snap)
     ok_local = bool(np.array_equal(res["ask"], want["ask"]) and np.array_equal(res["node"], want["node"])
                     and np.array_equal(res_e["ask"], want["ask"]) and np.array_equal(res_e["node"], want["node"]))
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name in ("ask", "node"):      # uint32 ids: exact in float64
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), res[name].astype(np.float64))
 
     def agg(seconds, allocations, ok):
         """whole-job numbers: allocations of all ranks / max time over ranks; every rank identical to its oracle"""
