@@ -1547,7 +1547,12 @@ int run_lattice(yk_engine* e, Cycle& c, bool& handoff) {
         } else {
             rc = lt_batch(e, B, ins);
             if (rc) return rc;
-            if (first && e->h_flag[0]) return e->fail(YK_ERR_RANGE, "NaN node score (zero total on a weighted resource)");
+            if (first && e->h_flag[0]) {
+                // the batch was decided on an order holding a NaN key and none of it is returned: the node records it
+                // changed must not be exported, so the tables keep what they held before the cycle
+                e->lt_active = false;
+                return e->fail(YK_ERR_RANGE, "NaN node score (zero total on a weighted resource)");
+            }
             status = e->h_lt_hdr[yklt::H_STATUS];
             consumed = (size_t)e->h_lt_hdr[yklt::H_CONSUMED];
             if (status == yklt::ST_NAN) return e->fail(YK_ERR_RANGE, "NaN node score after commit");
